@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- frames/s of MaskFusion::processFrame on a synthetic 640x480 .klg replay.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A step is one processFrame call (one pass of the per-frame dense hot path) on one frame of a seeded synthetic replay.
 
@@ -25,6 +25,13 @@ N > 1  (torchrun) workload = configs[3]: ONE 640x480 replay with 8 tracked objec
   value : frames/s, inputs resident in rank 0's HBM; e2e: the same with pinned host inputs on rank 0 and the pose read back
   single_process_same_workload : the same replay through one context on rank 0's GPU (the baseline the sharding is measured against)
   replicas : secondary leg, N independent configs[1] replays (the -static path has one model and does not shard)
+
+--dump-outputs DIR (N = 1): after the timed passes, what the last processFrame call left for its caller is written as DIR/<name>.npy
+(float32 / float64, ~40 MB): the background pose and pose log, the surfel count and a fixed seeded sample of the surfel store's rows,
+and the predicted view.  The replay and the pre-populated store are seeded, so two builds run with the same arguments can be
+compared output for output.
+
+Nothing is written into the tree (it may be read-only): no bytecode caches, the replay file goes to the temporary directory.
 """
 from __future__ import annotations
 
@@ -33,6 +40,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -40,10 +48,12 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True
 
 W, H = 640, 480
 CAPACITY = 2176 * 2176            # 64*floor(sqrt(5e6)/64) squared, Model.cpp:101-106
 PREPOP = 4_300_000                # dense room surfels uploaded after frame 0 (+ ~0.3M from the frame itself)
+DUMP_ROWS = 1 << 19               # surfel rows kept by --dump-outputs (24 MB of the ~230 MB store)
 METRIC = "frames/sec on 640x480 .klg replay"
 
 
@@ -115,7 +125,8 @@ def make_replay(n_frames, seed):
     for t in range(n_frames):
         r, _, _, _, d = sc.render(t)
         rgb[t], d16[t] = r, d
-    path = f"/tmp/mfb200_bench_{os.getpid()}.klg"
+    fd, path = tempfile.mkstemp(prefix="mfb200_bench_", suffix=".klg")
+    os.close(fd)
     mfb.write_klg(path, np.arange(n_frames + 1, dtype=np.int64) * 33333, d16, rgb)     # +1: hasMore() never yields the last frame (N11)
     rd = mfb.KlgLogReader(path, W, H)
     frames = []
@@ -176,7 +187,23 @@ def ncu_traffic(kernel):
     return int(tot), os.path.basename(files[-1])
 
 
-def static_leg(torch, mfb, stream, local, rank, world, K, Wm):
+def dump_outputs(mf, out_dir):
+    """what the last processFrame call left for its caller: pose, pose log, the surfel store (DUMP_ROWS rows at seeded positions when it
+    holds more) and the predicted view (splat image, vertex, normal, time)"""
+    gm = mf.getBackgroundModel()
+    surfels = gm.downloadMap()
+    if len(surfels) > DUMP_ROWS:
+        surfels = surfels[np.sort(np.random.default_rng(0).choice(len(surfels), DUMP_ROWS, replace=False))]
+    image, vertex, normal, stamp = gm.prediction()
+    arrays = {"pose": gm.getPose(), "pose_log": gm.poseLog(), "surfel_count": np.array([gm.lastCount()], np.float64), "surfels": surfels,
+              "prediction_image": image.astype(np.float32), "prediction_vertex": vertex, "prediction_normal": normal,
+              "prediction_time": stamp.astype(np.float32)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def static_leg(torch, mfb, stream, local, rank, world, K, Wm, dump_dir=None):
     """configs[1]: the main line at N = 1, the `replicas` leg at N > 1"""
     n_need = 1 + 3 * (Wm + K) + 2
     sc, frames = make_replay(n_need, seed=rank)
@@ -233,6 +260,8 @@ def static_leg(torch, mfb, stream, local, rank, world, K, Wm):
     stages = mf.stageTimes()
     mf.setProfiling(False)
     S_live = mf.getBackgroundModel().lastCount()
+    if dump_dir:
+        dump_outputs(mf, dump_dir)
     ms_all = sorted(r[0] for r in dev_runs)
     ms_dev, launches = ms_all[1], dev_runs[0][1]           # median of three passes
     if world > 1:
@@ -408,7 +437,7 @@ def run_ours(args, rank, world):
     torch.cuda.set_stream(stream)
     if world > 1:
         return run_sharded(args, rank, world, torch, mfb, stream, local, pre)
-    st = static_leg(torch, mfb, stream, local, rank, world, K, Wm)
+    st = static_leg(torch, mfb, stream, local, rank, world, K, Wm, dump_dir=args.dump_outputs)
     P = W * H
     fps = K / (st["ms_dev"] / 1e3)
     fps_e2e = K / (st["ms_e2e"] / 1e3)
@@ -689,8 +718,13 @@ def main():
     ap.add_argument("--steps", type=int, default=200)
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="ours")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy (N = 1)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", 0)); world = int(os.environ.get("WORLD_SIZE", 1))
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (world > 1 or args.impl != "ours"):
+        ap.error("--dump-outputs applies to the single-GPU run of this library")
     if args.impl == "reference":
         # the CPU arm uses all host threads it can, also under torchrun (which exports OMP_NUM_THREADS=1 for its workers)
         os.environ["OMP_NUM_THREADS"] = str(min(os.cpu_count() or 1, 32))

@@ -22,10 +22,22 @@ def detections(seed, H=48, W=64, N=6):
     return {"masks": masks, "scores": scores, "class_ids": class_ids, "rois": rois}
 
 
+def random_detections(rng, H=30, W=40):
+    """0-8 detections of scattered pixels, any score, class ids 1-4"""
+    N = int(rng.integers(0, 9))
+    return {"masks": (rng.random((H, W, N)) < 0.2), "scores": rng.uniform(0, 1, N).astype(np.float32),
+            "class_ids": rng.integers(1, 5, N).astype(np.int32), "rois": rng.integers(0, 30, (N, 4)).astype(np.int32)}
+
+
 out = {}
-cases = [(0, 0.0, [], []), (1, 0.7, [], []), (2, 0.5, [1, 2, 3], []), (3, 0.4, [], [0, 0, 250, 0, 251, 0]), (4, 0.99, [], [])]
-for k, (seed, min_score, cf, sa) in enumerate(cases):
-    r = detections(seed)
+cases = [(detections(0), 0.0, [], []), (detections(1), 0.7, [], []), (detections(2), 0.5, [1, 2, 3], []),
+         (detections(3), 0.4, [], [0, 0, 250, 0, 251, 0]), (detections(4), 0.99, [], [])]
+rng = np.random.default_rng(99)
+for _ in range(20):
+    r = random_detections(rng)
+    cf = [1, 3] if rng.random() < 0.5 else []
+    cases.append((r, float(rng.uniform(0, 1)), cf, []))
+for k, (r, min_score, cf, sa) in enumerate(cases):
     img, cls, rois = helpers.generate_id_image(r, min_score, cf, sa)
     out[f"c{k}_masks"] = r["masks"].astype(np.uint8); out[f"c{k}_scores"] = r["scores"]; out[f"c{k}_class_ids"] = r["class_ids"]; out[f"c{k}_rois"] = r["rois"]
     out[f"c{k}_min_score"] = np.float64(min_score); out[f"c{k}_filter"] = np.array(cf, np.int32); out[f"c{k}_special"] = np.array(sa, np.int32)

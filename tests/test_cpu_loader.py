@@ -272,7 +272,7 @@ def test_decoders_match_committed_opencv_vectors(product_lib, tmp_path):
 def test_generate_id_image_matches_reference_python(product_lib):
     """Mask R-CNN post-processing (MaskRCNN/helpers.py:70-98) against vectors produced by importing the reference's own function
     (tests/golden/make_idimage_golden.py): score threshold, class filter,
-    special assignments, overwrite order, nothing exported"""
+    special assignments, overwrite order, nothing exported; five hand-made cases and twenty seeded random ones"""
     from maskfusion_b200.api import generate_id_image
     g = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "idimage_golden.npz"))
     for k in range(int(g["ncases"])):
@@ -281,20 +281,7 @@ def test_generate_id_image_matches_reference_python(product_lib):
         assert np.array_equal(img, g[f"c{k}_img"]), k
         assert cls == g[f"c{k}_out_cls"].tolist(), k
         assert np.array_equal(np.array(rois, np.int32).reshape(-1, 4), g[f"c{k}_out_rois"]), k
-    if os.path.isdir("/root/reference/Core/Segmentation/MaskRCNN"):            # live, when the reference tree is present
-        import sys
-        sys.path.insert(0, "/root/reference/Core/Segmentation/MaskRCNN")
-        import helpers
-        rng = np.random.default_rng(99)
-        for _ in range(20):
-            N = int(rng.integers(0, 9)); H, W = 30, 40
-            r = {"masks": (rng.random((H, W, N)) < 0.2), "scores": rng.uniform(0, 1, N).astype(np.float32),
-                 "class_ids": rng.integers(1, 5, N).astype(np.int32), "rois": rng.integers(0, 30, (N, 4)).astype(np.int32)}
-            cf = [1, 3] if rng.random() < 0.5 else []
-            ms = float(rng.uniform(0, 1))
-            a = helpers.generate_id_image(dict(r), ms, cf)
-            b = generate_id_image({**r, "masks": r["masks"].astype(np.uint8)}, ms, cf)
-            assert np.array_equal(a[0], b[0]) and a[1] == b[1] and [list(map(int, x)) for x in a[2]] == b[2]
+    assert int(g["ncases"]) == 25
 
 
 def test_dir_reader_reads_what_the_reference_writes(product_lib, tmp_path):
